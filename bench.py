@@ -113,6 +113,36 @@ def synthetic_images(n_sets, batch, seed, img=IMG):
     return [torch.rand(batch, 3, img, img, generator=g) for _ in range(n_sets)]
 
 
+DUMP_MAX_ELEMENTS = 1 << 20   # per output array of --dump-outputs
+DUMP_MAX_BYTES = 64 << 20     # all arrays of --dump-outputs together
+
+
+def dump_outputs(out_dir, outputs):
+    """Writes every tensor of ``outputs`` as ``out_dir/<name>.npy``: floating tensors as float32, integer and bool ones as
+    float64 (exact).  A tensor of more than DUMP_MAX_ELEMENTS elements is written flattened, as the elements at
+    DUMP_MAX_ELEMENTS sorted flat indices drawn from a generator seeded with 0: the same shape gives the same sample, so
+    the files of two builds compare element for element.  More than DUMP_MAX_BYTES in all raises before anything is
+    written."""
+    import numpy as np
+
+    arrays = {}
+    for name, t in outputs.items():
+        if t is None:
+            continue
+        t = t.detach()
+        if t.numel() > DUMP_MAX_ELEMENTS:
+            g = torch.Generator().manual_seed(0)
+            idx = torch.randint(t.numel(), (DUMP_MAX_ELEMENTS,), generator=g).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        arrays[name] = (t.float() if t.is_floating_point() else t.double()).cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes of outputs, more than {DUMP_MAX_BYTES}")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------
 # reference arm / cpu baseline / gpu-eager baseline: the oracle (a port of the pure-Python reference path)
 # ------------------------------------------------------------------------------------------------
@@ -316,12 +346,22 @@ def run_b200(args):
         sampler.start()
     lib.wvn_profile_enable(3 if args.profile_gemm else 1)   # CUDA events around the roofline kernel's launches
     l0 = lib.wvn_launch_count()
-    total_ms = timed(lambda k: step(dev_imgs[k % 3]), args.steps)
+    last = {}
+
+    def timed_step(k):
+        r = step(dev_imgs[k % 3])
+        if k == args.steps - 1:   # only the last result: earlier steps' outputs are freed as without the dump
+            last["r"] = r
+
+    total_ms = timed(timed_step, args.steps)
     launches = lib.wvn_launch_count() - l0
     prof_ms = (ctypes.c_float * 2)()
     prof_n = (ctypes.c_longlong * 2)()
     _C.check(lib.wvn_profile_collect(prof_ms, prof_n))
     lib.wvn_profile_enable(0)
+    if args.dump_outputs and rank == 0:
+        # the step's result dict (maps, segmentation, pooled rows, graph, tokens) and the train step's loss metrics
+        dump_outputs(args.dump_outputs, last["r"] | {"metrics": hp.te._trainer.metrics})
     e2e_ms = timed(step_e2e, args.steps, finish=drain_e2e)
     clocks = sampler.stop() if rank == 0 else None
 
@@ -462,7 +502,14 @@ def main():
     ap.add_argument("--ingest", default="f32", choices=["f32", "u8"],
                     help="frame format at the boundary: f32 = (B,3,H,W) float in [0,1] (the reference's boundary, "
                          "BASELINE.json); u8 = camera frames (B,H,W,3) uint8, ingest fused into the patch loader (SURVEY.md §8f)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last one as DIR/<name>.npy (float32 / float64; "
+                         "arrays above 2^20 elements as a fixed, seeded sample of them) to compare two builds")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.impl != "b200" or args.profile_only):
+        ap.error("--dump-outputs writes the timed steps of --impl b200 (not with --profile-only)")
     if args.impl == "reference":
         run_reference(args)
     else:

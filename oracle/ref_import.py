@@ -1,7 +1,7 @@
 """ORACLE helper — path-import of the reference's own torch-only modules.
 
-Only usable where ``/root/reference`` exists (the build container), i.e. by
-``tests/golden/make_golden.py`` and by tests marked ``needs_reference``.  A normal
+Only usable where the reference tree exists (``REF_ROOT``), i.e. by ``tests/golden/make_golden.py``,
+which stores what the reference computes as fixtures for the tests.  A normal
 ``import wild_visual_navigation`` fails here (pytorch_lightning / omegaconf / pandas are absent),
 so stub packages are registered and the individual files are loaded with importlib, exactly as
 SURVEY.md §8c describes.  Nothing is copied: the modules execute from the read-only tree.

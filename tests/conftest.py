@@ -10,19 +10,15 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA sm_100a device (run on the B200 box)")
-    config.addinivalue_line("markers", "needs_reference: needs /root/reference (build container only)")
 
 
 def pytest_collection_modifyitems(config, items):
     import torch
 
     has_gpu = torch.cuda.is_available()
-    has_ref = os.path.isdir("/root/reference/wild_visual_navigation")
     for item in items:
         if "gpu" in item.keywords and not has_gpu:
             item.add_marker(pytest.mark.skip(reason="no CUDA device"))
-        if "needs_reference" in item.keywords and not has_ref:
-            item.add_marker(pytest.mark.skip(reason="/root/reference not present"))
 
 
 @pytest.fixture(scope="session")

@@ -16,6 +16,8 @@ Fixtures
                     the reference's method sources executed from the reference file
   checkpoint_ref.pt a checkpoint as TraversabilityEstimator.save_checkpoint writes it, from the reference's classes
   tmp_state_dict.pt the weight hand-off file as wvn_learning_node.py:381-394 writes it (reference SimpleMLP + ConfidenceGenerator)
+  simple_mlp_ref_state.pt  state dict of a fresh reference SimpleMLP(16, [8, 4, 1], True), the model the hand-off
+                    file is loaded into
   segments.npz      reference SegmentExtractor on a synthetic map + the reference's shipped
                     known-answer assets/graph/{seg,center}.pt and graph.pt edge_index
   extract_stego.pt  reference FeatureExtractor.extract end to end (stego segmentation + stego features) over the
@@ -115,6 +117,13 @@ def make_handoff(ns):
     new_model_state_dict = model.state_dict()
     new_model_state_dict["confidence_generator"] = cg.get_dict()
     torch.save(new_model_state_dict, os.path.join(HERE, "tmp_state_dict.pt"))
+
+
+def make_reference_mlp_state(ns):
+    """State dict of a freshly built reference SimpleMLP(16, [8, 4, 1], True): the parameter names, order, shapes and
+    init values the reference's inference node loads a hand-off file into."""
+    torch.manual_seed(5)
+    torch.save(ns.SimpleMLP(16, [8, 4, 1], True).state_dict(), os.path.join(HERE, "simple_mlp_ref_state.pt"))
 
 
 def make_checkpoint(ns):
@@ -499,6 +508,7 @@ if __name__ == "__main__":
     make_confidence(ns)
     make_confidence_methods(ns)
     make_handoff(ns)
+    make_reference_mlp_state(ns)
     make_checkpoint(ns)
     make_supervision()
     make_image_projector()

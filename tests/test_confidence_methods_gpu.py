@@ -84,5 +84,10 @@ def test_confidence_state_in_checkpoint_roundtrip(tmp_path):
         te2.load_checkpoint(str(tmp_path / f"{method}.pt"))
         a, b = te._traversability_loss._confidence_generator, te2._traversability_loss._confidence_generator
         assert torch.equal(a.mean.data, b.mean.data) and torch.equal(a.var.data, b.var.data)
+        sa, sb = a.state_dict(), b.state_dict()
+        assert list(sa) == list(sb) and all(torch.equal(sa[k], sb[k]) for k in sa)   # the whole state, bit for bit
+        # the step's per-row loss_reco is summed with shared-memory float atomics, so two runs of it on the same state
+        # differ in the last bits; the confidence's slope 1 / (2 std) turns one ulp of loss_reco into ~1e-6
+        # (test_bench_path_gpu.py::test_padded_step_equals_compacted_step holds this output to the same 1e-5)
         c1, c2 = te._trainer.step(x, y, yv).clone(), te2._trainer.step(x, y, yv).clone()
-        assert torch.allclose(c1, c2, atol=1e-6)
+        assert torch.allclose(c1, c2, atol=1e-5)

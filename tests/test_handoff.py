@@ -3,10 +3,8 @@ the file the reference's learning node writes (golden ``tmp_state_dict.pt``, pro
 classes) and the reader's change-detection semantics (wvn_feature_extractor_node.py:407-446)."""
 import os
 
-import pytest
 import torch
 
-from oracle import ref_import
 from wild_visual_navigation_b200.model.simple_mlp import SimpleMLP
 from wild_visual_navigation_b200.utils import ConfidenceGenerator, read_tmp_state_dict, write_tmp_state_dict, TMP_STATE_DICT_NAME
 
@@ -48,17 +46,29 @@ def test_roundtrip_and_change_detection(tmp_path):
     assert not read_tmp_state_dict(dst_model, dst_cg, f)
 
 
-@pytest.mark.needs_reference
-def test_reference_classes_load_our_file(tmp_path):
-    if not ref_import.available():
-        pytest.skip("reference tree not present")
-    ns = ref_import.load()
+def _module_with_state(state_dict):
+    """A module whose parameters have exactly the names, order and values of ``state_dict``."""
+    root = torch.nn.Module()
+    for name, v in state_dict.items():
+        *path, leaf = name.split(".")
+        m = root
+        for p in path:
+            if not hasattr(m, p):
+                m.add_module(p, torch.nn.Module())
+            m = getattr(m, p)
+        m.register_parameter(leaf, torch.nn.Parameter(v.clone()))
+    return root
+
+
+def test_reference_classes_load_our_file(tmp_path, golden_dir):
+    """The reference's inference node loads the hand-off file into its SimpleMLP with ``load_state_dict(strict=False)``;
+    that model's parameter layout and init come from the reference's own class (golden ``simple_mlp_ref_state.pt``)."""
     model, cg = _pair(3)
     with torch.no_grad():
         cg.mean[0], cg.std[0] = 0.11, 0.07
     f = write_tmp_state_dict(model, cg, str(tmp_path))
     new_model_state_dict = torch.load(f, weights_only=False)
-    ref_model = ns.SimpleMLP(16, [8, 4, 1], True)
+    ref_model = _module_with_state(torch.load(os.path.join(golden_dir, "simple_mlp_ref_state.pt")))
     k = list(ref_model.state_dict().keys())[-1]
     assert k in new_model_state_dict and (ref_model.state_dict()[k] != new_model_state_dict[k]).any()
     ref_model.load_state_dict(new_model_state_dict, strict=False)
